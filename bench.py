@@ -12,6 +12,7 @@ is all-reduced ONCE at the end, inside the timed region.  Secondary leg (`finetu
 ddpm_train.py:437-469 on the ratio-0.3 network (imgs/s; fp32-grade and, separately, the bf16 tier of BASELINE configs[3]).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c3] [--batch B] [--no-graph]
+                  [--dump-outputs DIR]
 Under torchrun the usual RANK/LOCAL_RANK/WORLD_SIZE/MASTER_* env is used; rank 0 prints ONE JSON line.
 """
 import argparse
@@ -26,6 +27,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "taylor_score_unet_fwd_bwd_passes_per_sec"
@@ -118,6 +120,24 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+# gradient entries --dump-outputs writes: 32 MB of float32, which with the loss keeps a dump well under 64 MB
+DUMP_GRAD_SAMPLES = 1 << 23
+
+
+def dump_outputs(out_dir, model, loss):
+    """What a caller of the timed Taylor path holds after its last step: that step's loss (loss.npy) and the gradients accumulated in
+    Parameter.grad.  Those are 143 MB for C1 and more for C3 / C5, so grad_sample.npy holds a fixed sample of them: positions drawn
+    from a seeded generator in the concatenation of every .grad in named_parameters() order, sorted, so two builds are compared at the
+    same entries."""
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([p.grad.reshape(-1) for _, p in model.named_parameters()])
+    if flat.numel() > DUMP_GRAD_SAMPLES:
+        idx = torch.randint(flat.numel(), (DUMP_GRAD_SAMPLES,), generator=torch.Generator().manual_seed(0)).sort().values
+        flat = flat[idx.to(flat.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_sample.npy"), flat.float().cpu().numpy())
 
 
 def synth_batch(B, hw=32, seed_off=0):
@@ -391,7 +411,7 @@ def finetune_bench(args, rank, world, dev, barrier, compute="fp32"):
     clean, noise = torch.randn(B, 3, hw, hw, generator=g).to(dev), torch.randn(B, 3, hw, hw, generator=g).to(dev)
     t = torch.randint(0, 1000, (B // 2 + 1,), generator=g)
     t = torch.cat([t, 1000 - t - 1])[:B].to(dev)
-    K = max(3, min(args.steps, 10))
+    K = args.steps
     for _ in range(3):
         st.step(clean, noise, t)
     barrier()
@@ -441,7 +461,7 @@ def secondary_scoring_leg(cfg_key, args, rank, world, dev, barrier):
     clean, noise = synth_batch(B, hw, seed_off=100 * rank)
     model.zero_grad()
     sc = TaylorScorer(model, clean.to(dev), noise.to(dev), use_graph=not args.no_graph, **extra(B, dev))
-    K, Wm = max(3, min(args.steps, 8)), 3
+    K, Wm = args.steps, 3
     ts = [(rank + k * world) % 1000 for k in range(Wm + K)]
     for k in range(Wm):
         sc.step(ts[k])
@@ -549,6 +569,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, sc.loss)
     eager_launches = lib.dp_launch_count() - c_before
     gpu_launches = eager_launches if args.no_graph else launches_per_pass * args.steps
     # ---------------- end-to-end through host buffers (H2D batch each step, D2H loss each step)
@@ -695,7 +717,14 @@ def main():
     ap.add_argument("--profile-pass", action="store_true", help="run one eager pass inside cudaProfilerStart/Stop (ncu)")
     ap.add_argument("--no-finetune", action="store_true", help="skip the secondary finetune imgs/s legs")
     ap.add_argument("--no-c3", action="store_true", help="skip the secondary BASELINE-config-3 (LSUN-256) scoring leg of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and a fixed sample of the accumulated gradients as DIR/*.npy "
+                         "(float32); the inputs depend on the arguments only, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the device path computed: use it with --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch is None:
         args.batch = CONFIGS[args.config]["batch"]
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)

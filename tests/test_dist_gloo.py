@@ -151,7 +151,7 @@ def _acc_worker(rank, world, port, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
     torch.set_num_threads(1)
     from accelerate import Accelerator
-    acc = Accelerator(gradient_accumulation_steps=1, mixed_precision="no")
+    acc = Accelerator(gradient_accumulation_steps=1, mixed_precision="no", cpu=True)   # gloo on the host, also where GPUs are visible
     assert acc.num_processes == world and acc.process_index == rank and acc.is_main_process == (rank == 0)
     torch.manual_seed(0)
     model = torch.nn.Linear(4, 3)

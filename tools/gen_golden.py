@@ -14,6 +14,7 @@ Outputs (all small, committed):
     tests/golden/cifar_cfg1_s3.pt  same with 3 timesteps (fast CPU check of the oracle)
     tests/golden/finetune_tiny.pt  2 finetune steps on TINY (Adam + clip + EMA), dropout 0
     tests/golden/ddim_tiny.pt      DDIMPipeline samples (uniform/eta 0/10 steps, quad/eta 0.5/7 steps) on TINY
+    tests/golden/ddpm_prune_magnitude_tiny.json  what ddpm_prune.py, run unmodified on the compat names, printed and saved
 """
 import argparse
 import hashlib
@@ -556,13 +557,44 @@ def gen_ref_pickle():
     print("ref_pickle", os.path.getsize(os.path.join(OUT, "ref_pruned_small.pth")), sum(p.numel() for p in m.parameters()))
 
 
+def gen_prune_script():
+    """ddpm_prune.py run UNMODIFIED through tests/run_script_traced.py (compat/ first on sys.path, trace mode) as `--pruner magnitude
+    --pruning_ratio 0.3 --device cpu` on a saved seed-0 TINY pipeline.  Without a GPU the script stops at its hard-coded
+    `pipeline.to("cuda")` (ddpm_prune.py:144), after everything kept here: the #Params / #MACS lines it printed, the files it saved,
+    their JSON configs, and the shapes and digest of its whole-module pickle of the pruned UNet."""
+    import shutil
+    import subprocess
+    import tempfile
+    tmp = tempfile.mkdtemp()
+    src, dst = os.path.join(tmp, "tiny_cifar_pipeline"), os.path.join(tmp, "pruned")     # "cifar" in the path: 32x32 example inputs
+    torch.manual_seed(0)
+    dp.DDPMPipeline(unet=dp.UNet2DModel(**dp.TINY_TEST_CONFIG), scheduler=dp.DDPMScheduler(num_train_timesteps=1000)).save_pretrained(src)
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "diff-pruning_b200", "compat"), ROOT]))
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "run_script_traced.py"), os.path.join(ref_shim.REF, "ddpm_prune.py"),
+                        "--model_path", src, "--save_path", dst, "--pruner", "magnitude", "--pruning_ratio", "0.3", "--device", "cpu",
+                        "--batch_size", "2"], cwd=ROOT, env=env, capture_output=True, text=True)
+    assert r.returncode == 0 or "cuda" in r.stderr.lower(), r.stderr[-2000:]
+    printed = [l for l in r.stdout.splitlines() if l.startswith(("#Params", "#MACS"))]
+    files = sorted(os.path.relpath(os.path.join(d, f), dst) for d, _, fs in os.walk(dst) for f in fs)
+    describe = ("import hashlib, json, sys, torch, diffusers\nm = torch.load(sys.argv[1], map_location='cpu')\nh = hashlib.sha256()\n"
+                "for k, v in m.state_dict().items():\n    h.update(k.encode()); h.update(v.contiguous().numpy().tobytes())\n"
+                "print(json.dumps({'class': type(m).__name__, 'shapes': {k: list(v.shape) for k, v in m.state_dict().items()}, "
+                "'state_dict_sha256': h.hexdigest()}))")
+    pickle = json.loads(subprocess.run([sys.executable, "-c", describe, os.path.join(dst, "pruned", "unet_pruned.pth")], env=env,
+                                       capture_output=True, text=True, check=True).stdout)
+    json.dump({"printed": printed, "files": files, "configs": {f: json.load(open(os.path.join(dst, f))) for f in files if f.endswith(".json")},
+               "pruned_pickle": pickle}, open(os.path.join(OUT, "ddpm_prune_magnitude_tiny.json"), "w"), indent=1)
+    shutil.rmtree(tmp)
+    print("prune_script", printed, len(files), pickle["state_dict_sha256"][:16])
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--skip-cfg1", action="store_true")
     ap.add_argument("--only", default=None)
     a = ap.parse_args()
-    torch.set_num_threads(os.cpu_count())
-    jobs = {"ldm_tiny": gen_ldm_tiny, "exp_importance": gen_exp_importance, "ref_pickle": gen_ref_pickle, "lsun_struct": gen_lsun_struct, "lr": gen_lr, "ckpt": gen_ckpt, "ddim": gen_ddim, "tiny": gen_tiny, "blocks": gen_blocks, "finetune": gen_finetune, "cifar_fwd": gen_cifar_fwd,
+    torch.set_num_threads(8)     # tests/test_oracle_golden.py GOLDEN_THREADS: the oracle re-sums in the same order
+    jobs = {"prune_script": gen_prune_script, "ldm_tiny": gen_ldm_tiny, "exp_importance": gen_exp_importance, "ref_pickle": gen_ref_pickle, "lsun_struct": gen_lsun_struct, "lr": gen_lr, "ckpt": gen_ckpt, "ddim": gen_ddim, "tiny": gen_tiny, "blocks": gen_blocks, "finetune": gen_finetune, "cifar_fwd": gen_cifar_fwd,
             "cfg1_s3": gen_cfg1_s3, "cfg3_s3": gen_cfg3_s3, "cfg1": gen_cfg1}
     for name, fn in jobs.items():
         if a.only and name != a.only:
