@@ -73,6 +73,7 @@ _SIGS = {
     "dp_conv2d_dgrad": (C.c_int, [C.POINTER(ConvArgs), vp]),
     "dp_conv2d_wgrad": (C.c_int, [C.POINTER(ConvArgs), vp]),
     "dp_conv_splitk_workspace_floats": (i64, [C.POINTER(ConvArgs), C.c_int]),
+    "dp_conv_presplit_eligible": (C.c_int, [C.POINTER(ConvArgs)]),
     "dp_conv2d_wgrad_reduce": (C.c_int, [C.POINTER(WgradReduceArgs), vp]),
     "dp_pack_conv_weight": (C.c_int, [vp, i32, i32, i32, i32, vp, vp, vp]),
     "dp_pack_conv_weight_tc": (C.c_int, [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]),
@@ -95,6 +96,7 @@ _SIGS = {
     "dp_softmax_bwd": (C.c_int, [vp, vp, vp, i64, i32, vp, vp]),
     "dp_groupnorm_workspace_bytes": (C.c_size_t, [i32, i32, i32, i32]),
     "dp_groupnorm_fwd": (C.c_int, [C.POINTER(GnArgs), vp]),
+    "dp_groupnorm_fwd_split": (C.c_int, [C.POINTER(GnArgs), vp, i64, vp]),
     "dp_groupnorm_bwd": (C.c_int, [C.POINTER(GnArgs), vp]),
     "dp_groupnorm_bwd_param": (C.c_int, [C.POINTER(GnArgs), vp]),
     "dp_silu_fwd": (C.c_int, [vp, vp, i64, vp]),

@@ -38,13 +38,15 @@ extern "C" int dp_tc_available(void) {
 #endif
 }
 
+// DP_CONV_X_SPLIT (an operand only the tensor-core kernels read) never falls back to the SIMT path
 extern "C" int dp_conv2d_fprop(const dp_conv_args* a, dp_stream_t s) {
 #ifdef DPB200_HAVE_TC
   if (a && !(a->flags & DP_CONV_FORCE_SIMT)) {
     int rc = dp_conv2d_fprop_tc(a, s);
-    if (rc != DP_ERR_UNSUPPORTED) return rc;
+    if (rc != DP_ERR_UNSUPPORTED || (a->flags & DP_CONV_X_SPLIT)) return rc;
   }
 #endif
+  if (a && (a->flags & DP_CONV_X_SPLIT)) return DP_ERR_UNSUPPORTED;
   return dp_conv2d_fprop_simt(a, s);
 }
 extern "C" int dp_conv2d_dgrad(const dp_conv_args* a, dp_stream_t s) {
@@ -60,8 +62,9 @@ extern "C" int dp_conv2d_wgrad(const dp_conv_args* a, dp_stream_t s) {
 #ifdef DPB200_HAVE_TC
   if (a && !(a->flags & DP_CONV_FORCE_SIMT)) {
     int rc = dp_conv2d_wgrad_tc(a, s);
-    if (rc != DP_ERR_UNSUPPORTED) return rc;
+    if (rc != DP_ERR_UNSUPPORTED || (a->flags & DP_CONV_X_SPLIT)) return rc;
   }
 #endif
+  if (a && (a->flags & DP_CONV_X_SPLIT)) return DP_ERR_UNSUPPORTED;
   return dp_conv2d_wgrad_simt(a, s);
 }

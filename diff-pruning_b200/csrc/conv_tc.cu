@@ -61,6 +61,7 @@ struct TcParams {
   // (row = tile_m * 128 + TMEM lane, pitch ws_ld); splitk_epilogue_kernel sums the splits in fixed order and applies the epilogue
   int ksplit, it_per_split;
   float* ws; long long ws_split_stride; int ws_ld;
+  int ld_split;             // pre-split A (conv_tc_ps_kernel<false, true>): fp16 elements from a pixel's hi channels to its lo' channels
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -116,23 +117,6 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, ui
       "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
       ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc)
       : "memory");
-}
-// amax slot -> power-of-two scale.  E = biased exponent of the bound (|v| < 2^(E-126)), clamped so that both factors are normal floats;
-// up = 2^(140-E) brings the operand below 2^14 (fp16 overflows at 65504), dn = 2^(E-140) undoes it in the epilogue.
-__device__ __forceinline__ int amax_exponent(const uint32_t* slot) {
-  const int E = (int)((__ldg(slot) >> 23) & 0xFFu);
-  return min(max(E, 14), 254);
-}
-__device__ __forceinline__ float scale_up(int E) { return __uint_as_float((uint32_t)(267 - E) << 23); }
-__device__ __forceinline__ float scale_dn(int E) { return __uint_as_float((uint32_t)(E - 13) << 23); }
-constexpr float LO_SCALE = 2048.f, LO_UNSCALE = 1.f / 2048.f;   // lo' = lo * 2^11 keeps the residual in fp16's normal range
-// two scaled values -> packed fp16 hi pair and lo' pair (low half = first element = lower address)
-__device__ __forceinline__ void split2(float a, float b, uint32_t& h, uint32_t& l) {
-  const __half2 hh = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(hh);
-  const __half2 ll = __floats2half2_rn((a - hf.x) * LO_SCALE, (b - hf.y) * LO_SCALE);
-  h = *reinterpret_cast<const uint32_t*>(&hh);
-  l = *reinterpret_cast<const uint32_t*>(&ll);
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -190,10 +174,14 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {  
 //               a_lo' 32), so the epilogue drains the single set into registers first and hands it back before touching global memory.
 // launch_tc picks TS for long K loops (>= 9 stages per work item: the 3x3 convolutions, + 7-15 % on the big layers) and the
 // double-buffered SS form for short ones (1x1 convolutions / linears: 4-stage tiles lose more to the accumulator hand-over than they gain).
+//   PRE = true  (TS = false) the A operand arrives split (DP_CONV_X_SPLIT, written by dp_groupnorm_fwd_split): TMA loads the hi box
+//               and the lo' box ([128 px][64 ch] fp16, SWIZZLE_128B — the layout the in-place split leaves) into the same two 16 KB
+//               slots, the MMA warp waits on the TMA barrier directly and the splitter warps idle.  A stage's chain is TMA -> MMA;
+//               the double-buffered SS accumulators, as there is no hand-over to avoid.
 constexpr int PS_THREADS = 320, PS_STAGES = 3;
 constexpr int PS_TS_MIN_STAGES = 9;     // K-loop length (stages per work item) from which the TS operand path wins
 
-template <bool TS>
+template <bool TS, bool PRE>
 __global__ void __launch_bounds__(PS_THREADS, 1)
 conv_tc_ps_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapBh,
                   const __grid_constant__ CUtensorMap mapBl, const TcParams p, const int tiles_m, const int total_tiles) {
@@ -258,8 +246,13 @@ conv_tc_ps_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
           const int tap = it / p.kchunks, kc = it - tap * p.kchunks;
           const uint32_t st = sbase + s * STAGE_BYTES;
           const int aw = q0 * p.in_stride + p.dw[tap], ah = p0 * p.in_stride + p.dh[tap];
-          tma_load_4d(st, &mapA, full_bar(s), kc * BK, aw, ah, n0);
-          tma_load_4d(st + A_BYTES, &mapA, full_bar(s), kc * BK + 32, aw, ah, n0);     // past the last channel: TMA zero fill
+          if constexpr (PRE) {       // hi channels [64 kc, 64 kc + 64) and their lo' at + ld_split (past the row: TMA zero fill)
+            tma_load_4d(st, &mapA, full_bar(s), kc * BK, aw, ah, n0);
+            tma_load_4d(st + A_BYTES, &mapA, full_bar(s), p.ld_split + kc * BK, aw, ah, n0);
+          } else {
+            tma_load_4d(st, &mapA, full_bar(s), kc * BK, aw, ah, n0);
+            tma_load_4d(st + A_BYTES, &mapA, full_bar(s), kc * BK + 32, aw, ah, n0);     // past the last channel: TMA zero fill
+          }
           const int tapb = p.b_from_img ? n0 : p.wt[tap];
           tma_load_3d(st + 2 * A_BYTES, &mapBh, full_bar(s), kc * BK, nblk * BN, tapb);
           tma_load_3d(st + 2 * A_BYTES + B_BYTES, &mapBl, full_bar(s), kc * BK, nblk * BN, tapb);
@@ -308,7 +301,7 @@ conv_tc_ps_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
           for (int it = it0; it < it1; ++it, ++g) {
             const int s = g % PS_STAGES;
             const uint32_t ph = (g / PS_STAGES) & 1u;
-            mbar_wait(conv_bar(s), ph);
+            mbar_wait(PRE ? full_bar(s) : conv_bar(s), ph);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const uint32_t st = sbase + s * STAGE_BYTES;
   #pragma unroll
@@ -328,7 +321,9 @@ conv_tc_ps_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
       }
     }
   } else if (warp < 6) {
-    if constexpr (TS) {
+    if constexpr (PRE) {
+      // ---- nothing to split
+    } else if constexpr (TS) {
       // ---- splitter warps 2..5 (TMEM lane quarter = warp & 3)
       const int r = (warp & 3) * 32 + lane;            // pixel row of the tile = TMEM lane
       const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
@@ -621,6 +616,7 @@ struct WgParams {
   int in_stride;             // x pixel = in_stride * dy pixel + tap offset
   const uint32_t* amax_x; const uint32_t* amax_y;
   float* bias_ws;            // optional [splits][K]: column sums of dy over this split's pixels (written by the tap 0 / c-tile 0 CTAs)
+  int ld_split;              // pre-split x (wgrad_tc_kernel<true>): fp16 elements from a pixel's hi channels to its lo' channels
 };
 constexpr int WG_KPIX = 64;                  // pixels per stage
 constexpr int WG_BLK = WG_KPIX * 128;        // 8 KB: one raw fp32 box [64 px][32 ch] = one fp16 block [64 px][64 ch]
@@ -636,7 +632,10 @@ __device__ __forceinline__ uint64_t umma_desc_mn(uint32_t saddr) {
 // 0..31 / 32..63 of dy, first / second raw box of every x row) + epilogue.  The ring is latency bound — period ~ (TMA latency + split +
 // MMA) / stages, r02_experiments.md section 13 — so halving the ~850-instruction split of a stage shortens every stage's chain; groups on
 // ALTERNATE stages did not (same chain) and, visiting each barrier only every second phase of a 3-stage ring, could be lapped.
+// PRE = true: x arrives split (DP_CONV_X_SPLIT): TMA loads its hi / lo' [64 px][64 ch] fp16 boxes straight into the x_hi / x_lo'
+// blocks, and the splitters only split dy.
 constexpr int WG_THREADS = 352;
+template <bool PRE>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant__ CUtensorMap mapX, const WgParams p) {
   constexpr int WSTAGES = WG_STAGES;
@@ -681,6 +680,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant
   // 32-channel boxes that hold valid channels (pruned widths: 96 / 179 / 358 ...): boxes past the last channel are neither loaded nor
   // split — their accumulator rows / columns are never stored, so whatever the stage buffers still hold there is harmless
   const int dy_boxes = min(4, (p.K - kt * 128 + 31) >> 5), x_boxes = min(4, (p.C - ct * 128 + 31) >> 5);
+  const int x_blocks = min(2, (p.C - ct * 128 + 63) >> 6);    // pre-split x: 64-channel hi / lo' block pairs holding valid channels
 
   if (warp == 0) {
     if (lane == 0) {
@@ -690,7 +690,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant
         const int s = it % WSTAGES;
         const uint32_t ph = (uint32_t)(it / WSTAGES) & 1u;
         mbar_wait(empty_bar(s), ph ^ 1u);
-        mbar_expect_tx(full_bar(s), (uint32_t)((dy_boxes + x_boxes) * WG_BLK));
+        mbar_expect_tx(full_bar(s), (uint32_t)((dy_boxes + (PRE ? 2 * x_blocks : x_boxes)) * WG_BLK));
         const int chunk = chunk0 + it;
         const int tw = chunk % p.tiles_w;
         const int th = (chunk / p.tiles_w) % p.tiles_h;
@@ -702,9 +702,16 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant
         for (int b = 0; b < 4; ++b)     // dy: up to 4 boxes of 32 out-channels
           if (b < dy_boxes) tma_load_4d(st + b * WG_BLK, &mapDy, full_bar(s), kt * 128 + b * 32, q0, p0, n0);
 #pragma unroll
-        for (int j = 0; j < 2; ++j) {   // x: channels [64j, 64j+32) -> future x_hi[j], [64j+32, 64j+64) -> future x_lo'[j]
-          if (2 * j < x_boxes) tma_load_4d(st + (4 + j) * WG_BLK, &mapX, full_bar(s), ct * 128 + 64 * j, xw, xh, n0);
-          if (2 * j + 1 < x_boxes) tma_load_4d(st + (6 + j) * WG_BLK, &mapX, full_bar(s), ct * 128 + 64 * j + 32, xw, xh, n0);
+        for (int j = 0; j < 2; ++j) {
+          if constexpr (PRE) {          // x: hi channels [64j, 64j+64) -> x_hi[j], their lo' -> x_lo'[j]
+            if (j < x_blocks) {
+              tma_load_4d(st + (4 + j) * WG_BLK, &mapX, full_bar(s), ct * 128 + 64 * j, xw, xh, n0);
+              tma_load_4d(st + (6 + j) * WG_BLK, &mapX, full_bar(s), p.ld_split + ct * 128 + 64 * j, xw, xh, n0);
+            }
+          } else {                      // x: channels [64j, 64j+32) -> future x_hi[j], [64j+32, 64j+64) -> future x_lo'[j]
+            if (2 * j < x_boxes) tma_load_4d(st + (4 + j) * WG_BLK, &mapX, full_bar(s), ct * 128 + 64 * j, xw, xh, n0);
+            if (2 * j + 1 < x_boxes) tma_load_4d(st + (6 + j) * WG_BLK, &mapX, full_bar(s), ct * 128 + 64 * j + 32, xw, xh, n0);
+          }
         }
       }
     }
@@ -778,7 +785,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant
       }
       // (2) x: row xp of block xj.  This thread reads the row's raw box `half` (channels 32 half .. 32 half + 31 of the block); once BOTH
       //     halves have read, it writes chunks 4 half .. 4 half + 3 of the fp16 x_hi row (over box 0) and of the x_lo' row (over box 1)
-      {
+      if constexpr (!PRE) {
         uint8_t* a0 = smem + s * STAGE_BYTES + (4 + xj) * WG_BLK + xp * 128;
         uint8_t* a1 = a0 + 2 * WG_BLK;
         const uint8_t* src = half ? a1 : a0;
@@ -875,9 +882,11 @@ int tc_init() {
   if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
       qres != cudaDriverEntryPointSuccess) { (void)cudaGetLastError(); return 0; }
   g_encode = (EncodeTiledFn)fn;
-  bool ok = cudaFuncSetAttribute(conv_tc_ps_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PS_SMEM) == cudaSuccess;
-  ok = ok && cudaFuncSetAttribute(conv_tc_ps_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PS_SMEM) == cudaSuccess;
-  ok = ok && cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM) == cudaSuccess;
+  bool ok = cudaFuncSetAttribute(conv_tc_ps_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PS_SMEM) == cudaSuccess;
+  ok = ok && cudaFuncSetAttribute(conv_tc_ps_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PS_SMEM) == cudaSuccess;
+  ok = ok && cudaFuncSetAttribute(conv_tc_ps_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PS_SMEM) == cudaSuccess;
+  ok = ok && cudaFuncSetAttribute(wgrad_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM) == cudaSuccess;
+  ok = ok && cudaFuncSetAttribute(wgrad_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM) == cudaSuccess;
   cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
   if (!ok) { (void)cudaGetLastError(); return 0; }
   (void)cudaGetLastError();
@@ -931,16 +940,19 @@ static int pick_ksplit(int tiles, int iters, int& it_per_split) {
 
 // Shared launcher.  act: [Nimg][H][W][Kg] fp32 view (ld_act) = A operand on whose pixel grid the M tiles live, amax_a its amax slot;
 // w_hi / w_lo: fp16 [T][Nout][ldb] with the scale of slot amax_b; out: [Nimg][Ho][Wo][Nout] view, output pixel = (p*os+oa, q*os+ob).
-// ws: optional split-K workspace (dp_conv_splitk_workspace_floats floats); *ws_need != nullptr: only report the floats a split launch needs
+// ws: optional split-K workspace (dp_conv_splitk_workspace_floats floats); *ws_need != nullptr: only report the floats a split launch needs.
+// act_split: the A operand already split (DP_CONV_X_SPLIT layout, hi -> lo' distance ld_split fp16 elements): read instead of act
 int launch_tc(const float* act, long long ld_act, const uint32_t* amax_a, int Nimg, int H, int W, int Kg, const void* w_hi, const void* w_lo,
               const uint32_t* amax_b, int Nout, int T, const TapTable& taps, int os, int oa, int ob, int Ho, int Wo, float* out,
               long long ld_out, const float* bias, const float* rowadd, long long ld_rowadd, const float* residual, long long ld_res,
               int accumulate, cudaStream_t st, float alpha = 1.0f, int b_from_img = 0, int in_stride = 1, int ldb = -1, float* ws = nullptr,
-              long long* ws_need = nullptr, uint32_t* amax_out = nullptr) {
+              long long* ws_need = nullptr, uint32_t* amax_out = nullptr, const void* act_split = nullptr, long long ld_split = 0) {
   if (ldb < 0) ldb = wrow(Kg);   // packed conv weights; batched GEMM callers pass their own row pitch
   if (!tc_init()) return DP_ERR_UNSUPPORTED;
   if (!ws_need && (!w_hi || !w_lo || !amax_a || !amax_b)) return DP_ERR_UNSUPPORTED;
-  if (!ws_need && (ld_act % 4 || ((uintptr_t)act & 15) || ((uintptr_t)w_hi & 15) || ((uintptr_t)w_lo & 15))) return DP_ERR_UNSUPPORTED;
+  if (!ws_need && !act_split && (ld_act % 4 || ((uintptr_t)act & 15))) return DP_ERR_UNSUPPORTED;
+  if (!ws_need && (((uintptr_t)w_hi & 15) || ((uintptr_t)w_lo & 15))) return DP_ERR_UNSUPPORTED;
+  if (act_split && (in_stride != 1 || ld_split < Kg || ld_split % 8 || ((uintptr_t)act_split & 15))) return DP_ERR_UNSUPPORTED;
   int bw, bh, bn;
   if (!pick_box(Nimg, H, W, bw, bh, bn)) return DP_ERR_UNSUPPORTED;
   constexpr int BN = 128;
@@ -963,7 +975,12 @@ int launch_tc(const float* act, long long ld_act, const uint32_t* amax_a, int Ni
     cuuint64_t str[3] = {(cuuint64_t)ld_act * 4, Win * ld_act * 4, Hin * Win * ld_act * 4};
     cuuint32_t box[4] = {32u, (cuuint32_t)(bw * in_stride), (cuuint32_t)(bh * in_stride), (cuuint32_t)bn};   // two boxes of 32 fp32 channels per stage
     if (box[1] > 256 || box[2] > 256) return DP_ERR_UNSUPPORTED;
-    if (!make_map(&mA, act, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, in_stride)) return DP_ERR_UNSUPPORTED;
+    if (act_split) {   // [pixel][hi | lo'] fp16 rows of 2 ld_split elements: boxes of 64 channels (128 bytes)
+      cuuint64_t sdims[4] = {(cuuint64_t)(2 * ld_split), Win, Hin, (cuuint64_t)Nimg};
+      cuuint64_t sstr[3] = {(cuuint64_t)ld_split * 4, Win * ld_split * 4, Hin * Win * ld_split * 4};
+      box[0] = (cuuint32_t)BK;
+      if (!make_map(&mA, act_split, 4, sdims, sstr, box, CU_TENSOR_MAP_SWIZZLE_128B, 1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16)) return DP_ERR_UNSUPPORTED;
+    } else if (!make_map(&mA, act, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, in_stride)) return DP_ERR_UNSUPPORTED;
   }
   {
     const cuuint64_t Kp = (cuuint64_t)ldb;
@@ -989,6 +1006,7 @@ int launch_tc(const float* act, long long ld_act, const uint32_t* amax_a, int Ni
   const int tiles_n = (Nimg + bn - 1) / bn;
   dim3 grid((unsigned)(p.tiles_w * p.tiles_h * tiles_n), (unsigned)((Nout + BN - 1) / BN));
   p.ksplit = 1; p.it_per_split = p.ntaps * p.kchunks;
+  p.ld_split = (int)ld_split;
   {
     const int tiles_m = (int)grid.x, total = (int)(grid.x * grid.y);
     if (ws && !b_from_img) {
@@ -997,8 +1015,9 @@ int launch_tc(const float* act, long long ld_act, const uint32_t* amax_a, int Ni
     }
     const int work = total * p.ksplit;
     const int ctas = work < g_num_sms ? work : g_num_sms;
-    if (p.it_per_split >= PS_TS_MIN_STAGES) conv_tc_ps_kernel<true><<<ctas, PS_THREADS, PS_SMEM, st>>>(mA, mBh, mBl, p, tiles_m, total);
-    else conv_tc_ps_kernel<false><<<ctas, PS_THREADS, PS_SMEM, st>>>(mA, mBh, mBl, p, tiles_m, total);
+    if (act_split) conv_tc_ps_kernel<false, true><<<ctas, PS_THREADS, PS_SMEM, st>>>(mA, mBh, mBl, p, tiles_m, total);
+    else if (p.it_per_split >= PS_TS_MIN_STAGES) conv_tc_ps_kernel<true, false><<<ctas, PS_THREADS, PS_SMEM, st>>>(mA, mBh, mBl, p, tiles_m, total);
+    else conv_tc_ps_kernel<false, false><<<ctas, PS_THREADS, PS_SMEM, st>>>(mA, mBh, mBl, p, tiles_m, total);
     if (p.ksplit > 1) {
       int rc = dp_check_launch();
       if (rc) return rc;
@@ -1204,16 +1223,17 @@ static TapTable dense_taps(int R, int S, int pad, bool flip) {
 
 int dp_conv2d_fprop_tc(const dp_conv_args* a, dp_stream_t stream) {
   if (!a || !a->x || !a->y) return DP_ERR_UNSUPPORTED;   // let the SIMT entry produce the precise error
+  const bool pre = (a->flags & DP_CONV_X_SPLIT) != 0;
   if (a->R != a->S || (a->R != 1 && a->R != 3) || a->pad_l != a->pad_t) return DP_ERR_UNSUPPORTED;
   // stride 1: 'same' padding.  stride 2: 3x3 with pad 1, or pad 0 + the (0,1,0,1) zero border of Downsample2D (resnet.py:213-218) which
   // TMA out-of-bounds zero fill provides for free
   if (!((a->stride == 1 && a->pad_t == (a->R - 1) / 2) || (a->stride == 2 && a->R == 3 && (a->pad_t == 0 || a->pad_t == 1)))) return DP_ERR_UNSUPPORTED;
   if (a->P * a->stride != a->H || a->Q * a->stride != a->W) return DP_ERR_UNSUPPORTED;   // stride 2: even extents, out = in / 2 (Downsample2D, pad 1)
-  if (a->N <= 0 || a->H <= 0 || a->W <= 0 || a->C <= 0 || a->K <= 0 || a->ldx < a->C || a->ldy < a->K) return DP_ERR_UNSUPPORTED;
-  return launch_tc((const float*)a->x, a->ldx, a->amax_x, a->N, a->P, a->Q, a->C, a->w_tc_hi, a->w_tc_lo, a->amax_w, a->K, a->R * a->S,
-                   dense_taps(a->R, a->S, a->pad_t, false), 1, 0, 0, a->P, a->Q, (float*)a->y, a->ldy, a->bias, a->rowadd,
+  if (a->N <= 0 || a->H <= 0 || a->W <= 0 || a->C <= 0 || a->K <= 0 || (!pre && a->ldx < a->C) || a->ldy < a->K) return DP_ERR_UNSUPPORTED;
+  return launch_tc(pre ? nullptr : (const float*)a->x, a->ldx, a->amax_x, a->N, a->P, a->Q, a->C, a->w_tc_hi, a->w_tc_lo, a->amax_w, a->K,
+                   a->R * a->S, dense_taps(a->R, a->S, a->pad_t, false), 1, 0, 0, a->P, a->Q, (float*)a->y, a->ldy, a->bias, a->rowadd,
                    a->ld_rowadd, a->residual, a->ld_res, (a->flags & DP_CONV_ACCUMULATE) ? 1 : 0, (cudaStream_t)stream, 1.0f, 0, a->stride, -1,
-                   a->workspace, nullptr, a->amax_out);
+                   a->workspace, nullptr, a->amax_out, pre ? a->x : nullptr, pre ? a->ldx : 0);
 }
 
 // stride-1 dgrad == fprop of dy with the taps flipped and the (K,C) roles swapped: dx[n,h,w,c] = sum dy[n,h+1-r,w+1-s,k] W[k,c,r,s].
@@ -1301,7 +1321,10 @@ int dp_conv2d_wgrad_tc(const dp_conv_args* a, dp_stream_t stream) {
   // TMA out-of-bounds zero fill provides for free
   if (!((a->stride == 1 && a->pad_t == (a->R - 1) / 2) || (a->stride == 2 && a->R == 3 && (a->pad_t == 0 || a->pad_t == 1)))) return DP_ERR_UNSUPPORTED;
   if (a->P * a->stride != a->H || a->Q * a->stride != a->W || a->splits < 1) return DP_ERR_UNSUPPORTED;
-  if (a->ldx % 4 || a->ldy % 4 || ((uintptr_t)a->x & 15) || ((uintptr_t)a->y & 15)) return DP_ERR_UNSUPPORTED;
+  const bool pre = (a->flags & DP_CONV_X_SPLIT) != 0;
+  if (a->ldy % 4 || ((uintptr_t)a->y & 15)) return DP_ERR_UNSUPPORTED;
+  if (!pre && (a->ldx % 4 || ((uintptr_t)a->x & 15))) return DP_ERR_UNSUPPORTED;
+  if (pre && (a->stride != 1 || a->ldx < a->C || a->ldx % 8 || ((uintptr_t)a->x & 15))) return DP_ERR_UNSUPPORTED;
   int bw, bh, bn;
   if (!a->amax_x || !a->amax_y) return DP_ERR_UNSUPPORTED;
   if (!pick_box64(a->P, a->Q, bw, bh, bn)) return DP_ERR_UNSUPPORTED;   // 64-pixel chunks of the dy (output) grid; images past the batch
@@ -1313,7 +1336,12 @@ int dp_conv2d_wgrad_tc(const dp_conv_args* a, dp_stream_t stream) {
     cuuint32_t box[4] = {32, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bn};
     if (!make_map(&mDy, a->y, 4, dims, str, box)) return DP_ERR_UNSUPPORTED;
   }
-  {   // x is sampled at stride * (output pixel) + tap offset: TMA element strides on W, H
+  if (pre) {   // [pixel][hi | lo'] fp16 rows of 2 ldx elements: [64 px][64 ch] boxes
+    cuuint64_t dims[4] = {(cuuint64_t)(2 * a->ldx), (cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->N};
+    cuuint64_t str[3] = {(cuuint64_t)a->ldx * 4, (cuuint64_t)a->W * a->ldx * 4, (cuuint64_t)a->H * a->W * a->ldx * 4};
+    cuuint32_t box[4] = {64, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bn};
+    if (!make_map(&mX, a->x, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, 1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16)) return DP_ERR_UNSUPPORTED;
+  } else {   // x is sampled at stride * (output pixel) + tap offset: TMA element strides on W, H
     cuuint64_t dims[4] = {(cuuint64_t)a->C, (cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->N};
     cuuint64_t str[3] = {(cuuint64_t)a->ldx * 4, (cuuint64_t)a->W * a->ldx * 4, (cuuint64_t)a->H * a->W * a->ldx * 4};
     cuuint32_t box[4] = {32, (cuuint32_t)(bw * a->stride), (cuuint32_t)(bh * a->stride), (cuuint32_t)bn};
@@ -1324,14 +1352,25 @@ int dp_conv2d_wgrad_tc(const dp_conv_args* a, dp_stream_t stream) {
   p.Nimg = a->N; p.H = a->P; p.W = a->Q; p.C = a->C; p.K = a->K; p.R = a->R; p.S = a->S; p.pad = a->pad_t; p.in_stride = a->stride;
   p.bw = bw; p.bh = bh; p.bn = bn; p.tiles_w = a->Q / bw; p.tiles_h = a->P / bh;
   p.total_chunks = p.tiles_w * p.tiles_h * img_boxes;
-  p.amax_x = a->amax_x; p.amax_y = a->amax_y; p.bias_ws = a->bias_ws;
+  p.amax_x = a->amax_x; p.amax_y = a->amax_y; p.bias_ws = a->bias_ws; p.ld_split = pre ? (int)a->ldx : 0;
   p.chunks_per_split = (p.total_chunks + a->splits - 1) / a->splits;
   p.c_tiles = (a->C + 127) / 128;
   p.ws = a->workspace;
   const int k_tiles = (a->K + 127) / 128;
   dim3 grid((unsigned)(k_tiles * p.c_tiles * a->R * a->S), (unsigned)a->splits);
-  wgrad_tc_kernel<<<grid, WG_THREADS, WG_SMEM, (cudaStream_t)stream>>>(mDy, mX, p);
+  if (pre) wgrad_tc_kernel<true><<<grid, WG_THREADS, WG_SMEM, (cudaStream_t)stream>>>(mDy, mX, p);
+  else wgrad_tc_kernel<false><<<grid, WG_THREADS, WG_SMEM, (cudaStream_t)stream>>>(mDy, mX, p);
   return dp_check_launch();
+}
+
+extern "C" int dp_conv_presplit_eligible(const dp_conv_args* a) {
+  if (!a || !tc_init()) return DP_ERR_UNSUPPORTED;
+  if (a->N <= 0 || a->H <= 0 || a->W <= 0 || a->C <= 0 || a->K <= 0) return DP_ERR_UNSUPPORTED;
+  if (a->R != a->S || (a->R != 1 && a->R != 3) || a->stride != 1 || a->pad_t != (a->R - 1) / 2 || a->pad_l != a->pad_t) return DP_ERR_UNSUPPORTED;
+  if (a->P != a->H || a->Q != a->W) return DP_ERR_UNSUPPORTED;
+  int bw, bh, bn;
+  if (!pick_box(a->N, a->H, a->W, bw, bh, bn) || !pick_box64(a->H, a->W, bw, bh, bn)) return DP_ERR_UNSUPPORTED;   // fprop / wgrad tiles
+  return DP_OK;
 }
 
 extern "C" int dp_pack_conv_weight_tc(const float* w, int32_t K, int32_t C, int32_t R, int32_t S, void* kc_hi, void* kc_lo,

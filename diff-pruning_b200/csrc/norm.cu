@@ -424,16 +424,47 @@ __global__ void __launch_bounds__(NT) gn_stats4_kernel(const dp_gn_args a, const
   }
 }
 
-__global__ void __launch_bounds__(NT, 4) gn_apply4_kernel(const dp_gn_args a, const Map mp, const double* __restrict__ fold_ws) {
+// Bound of |y| known before y exists, from gamma / beta alone (every block derives the same bits, on every launch: safe under graph
+// replay and after a weight update).  Over a group of n values |x - mean| <= sqrt(n - 1) * std (Samuelson) and rstd <= 1 / std, so
+// |x_hat| <= sqrt(n - 1) and |gn(x)| <= B = max|gamma| sqrt(n - 1) + max|beta|; |silu(v)| <= max(|v|, 0.2785); dropout scales by its
+// exact inverse keep rate.  Rounded up, plus 2^-10 for the fp32 rounding of the statistics and of the SiLU.  Block (0, 0) stores B as
+// the output's amax slot; the return value is the convolutions' operand scale for that slot.  Called by all threads of the block.
+__device__ float gn_split_scale(const dp_gn_args& a, const Drop& drop, int cpg) {
+  __shared__ float red[2][NT / 32];
+  float gm = 0.f, bm = 0.f;
+  for (int c = threadIdx.x; c < a.C; c += NT) { gm = fmaxf(gm, fabsf(__ldg(a.gamma + c))); bm = fmaxf(bm, fabsf(__ldg(a.beta + c))); }
+  gm = warp_max(gm); bm = warp_max(bm);
+  if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = gm; red[1][threadIdx.x >> 5] = bm; }
+  __syncthreads();
+  gm = 0.f; bm = 0.f;
+#pragma unroll
+  for (int w = 0; w < NT / 32; ++w) { gm = fmaxf(gm, red[0][w]); bm = fmaxf(bm, red[1][w]); }
+  const long long n = (long long)cpg * a.HW;
+  float B = __fmaf_ru(gm, __fsqrt_ru((float)(n - 1)), bm);
+  if (a.silu) B = fmaxf(B, 0.2785f);
+  if (drop.on) B = __fmul_ru(B, drop.inv);
+  B = __fmul_ru(B, 1.0f + 0x1p-10f);
+  const uint32_t bits = __float_as_uint(B);
+  if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) *a.amax_y = bits;
+  return scale_up(amax_exponent_bits(bits));
+}
+
+// SPLIT: also write the split output (dp_groupnorm_fwd_split).  Its own instantiation, with room for the extra live registers (at 4 blocks per SM it spilled)
+template <bool SPLIT>
+__global__ void __launch_bounds__(NT, SPLIT ? 3 : 4) gn_apply4_kernel(const dp_gn_args a, const Map mp, const double* __restrict__ fold_ws, __half* __restrict__ ysplit,
+                                                             const long long ldys) {
   extern __shared__ float shst[];   // folded finalize: [2][G]
   const int n = blockIdx.y, chunk = blockIdx.x, tid = threadIdx.x;
   const int ct = tid % mp.CT, pl = tid / mp.CT, c0 = ct * 4;
   const float* gmean = a.mean + n * a.G;
   const float* grstd = a.rstd + n * a.G;
   if (fold_ws) { gn_fold_stats(a, mp, fold_ws, n, chunk == 0, shst, shst + a.G); gmean = shst; grstd = shst + a.G; }
+  const Drop drop = make_drop(a);
+  const int cpg = a.C / a.G;
+  float ssplit = 0.f;       // split output: scale of the bound B, the same in every block
+  if constexpr (SPLIT) ssplit = gn_split_scale(a, drop, cpg);
   if (c0 >= a.C) return;
   const int p0 = chunk * mp.PPC, p1 = min(a.HW, p0 + mp.PPC);
-  const int cpg = a.C / a.G;
   float sc[4], shf[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
@@ -443,7 +474,7 @@ __global__ void __launch_bounds__(NT, 4) gn_apply4_kernel(const dp_gn_args a, co
   }
   const float* xb = a.x + (long long)n * a.HW * a.ldx + c0;
   float* yb = a.y + (long long)n * a.HW * a.ldy + c0;
-  const Drop drop = make_drop(a);
+  __half* ysb = ysplit + (long long)n * a.HW * 2 * ldys + c0;
   float amax = 0.f;
   float4 cur[GU], nxt[GU];       // software pipeline: see gn_stats4_kernel
   const int gstep = GU * mp.PL;
@@ -477,6 +508,14 @@ __global__ void __launch_bounds__(NT, 4) gn_apply4_kernel(const dp_gn_args a, co
       uint2 pk = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
       *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(a.y_bf16) + ((long long)n * a.HW + pix) * a.ldyb + c0) = pk;
     }
+    if constexpr (SPLIT) {  // the convolutions' hi / lo' operand pair, exactly what their splitter makes of y with the same scale (8-byte aligned)
+      uint2 h, l;
+      split2(y[0] * ssplit, y[1] * ssplit, h.x, l.x);
+      split2(y[2] * ssplit, y[3] * ssplit, h.y, l.y);
+      __half* dst = ysb + (long long)pix * 2 * ldys;
+      *reinterpret_cast<uint2*>(dst) = h;
+      *reinterpret_cast<uint2*>(dst + ldys) = l;
+    }
     amax = fmaxf(fmaxf(amax, fmaxf(fabsf(y[0]), fabsf(y[1]))), fmaxf(fabsf(y[2]), fabsf(y[3])));
    }
    if (more) {
@@ -484,7 +523,7 @@ __global__ void __launch_bounds__(NT, 4) gn_apply4_kernel(const dp_gn_args a, co
     for (int u = 0; u < GU; ++u) cur[u] = nxt[u];
    }
   }
-  if (a.amax_y) amax_commit(a.amax_y, amax);
+  if (a.amax_y && !SPLIT) amax_commit(a.amax_y, amax);
 }
 
 __global__ void __launch_bounds__(NT, 4) gn_bwd_partial4_kernel(const dp_gn_args a, const Map mp, float* __restrict__ part) {
@@ -777,14 +816,17 @@ static int gn_validate(const dp_gn_args* a) {
   return DP_OK;
 }
 
-extern "C" int dp_groupnorm_fwd(const dp_gn_args* a, dp_stream_t stream) {
+static int gn_fwd(const dp_gn_args* a, void* ysplit, int64_t ldys, dp_stream_t stream) {
   int rc = gn_validate(a);
   if (rc) return rc;
-  DP_REQUIRE(a->y || a->y_bf16, DP_ERR_NULL);
+  DP_REQUIRE(a->y || a->y_bf16 || ysplit, DP_ERR_NULL);
   DP_REQUIRE(!a->y || a->ldy >= a->C, DP_ERR_SHAPE);
   DP_REQUIRE(!a->y_bf16 || (a->ldyb >= a->C && a->ldyb % 8 == 0 && (((uintptr_t)a->y_bf16) & 15) == 0), DP_ERR_ALIGN);
+  DP_REQUIRE(!ysplit || a->amax_y, DP_ERR_NULL);
+  DP_REQUIRE(!ysplit || (ldys >= a->C && ldys % 8 == 0 && (((uintptr_t)ysplit) & 15) == 0), DP_ERR_ALIGN);
   cudaStream_t st = (cudaStream_t)stream;
   const bool v4 = (a->C % 4 == 0) && al16(a->x, a->ldx) && al16(a->y, a->ldy);
+  DP_REQUIRE(!ysplit || (v4 && !ln_fast(a)), DP_ERR_UNSUPPORTED);    // the split output is written by the float4 apply kernel only
   if (v4 && a->y && ln_fast(a) && al16(a->gamma, 0) && al16(a->beta, 0)) {     // LayerNorm over tokens: one warp per row
     ln_fwd_kernel<<<(unsigned)((a->N + 7) / 8), 256, 0, st>>>(*a);
     return dp_check_launch();
@@ -805,9 +847,16 @@ extern "C" int dp_groupnorm_fwd(const dp_gn_args* a, dp_stream_t stream) {
   }
   const double* fws = fold ? (const double*)a->workspace : nullptr;
   const size_t fsm = fold ? 2 * (size_t)a->G * sizeof(float) : 0;
-  if (v4) gn_apply4_kernel<<<grid, NT, fsm, st>>>(*a, mp, fws);
+  if (v4 && ysplit) gn_apply4_kernel<true><<<grid, NT, fsm, st>>>(*a, mp, fws, (__half*)ysplit, ldys);
+  else if (v4) gn_apply4_kernel<false><<<grid, NT, fsm, st>>>(*a, mp, fws, nullptr, 0);
   else gn_apply_kernel<<<grid, NT, fsm, st>>>(*a, mp, fws);
   return dp_check_launch();
+}
+
+extern "C" int dp_groupnorm_fwd(const dp_gn_args* a, dp_stream_t stream) { return gn_fwd(a, nullptr, 0, stream); }
+extern "C" int dp_groupnorm_fwd_split(const dp_gn_args* a, void* y_split, int64_t ldys, dp_stream_t stream) {
+  DP_REQUIRE(y_split, DP_ERR_NULL);
+  return gn_fwd(a, y_split, ldys, stream);
 }
 
 extern "C" int dp_groupnorm_bwd(const dp_gn_args* a, dp_stream_t stream) {

@@ -104,6 +104,10 @@ AUDIT_SLOTS = False  # tests: plans built while this is set check every amax slo
 SIDE_WGRAD = True  # backward: weight-gradient launches (wgrad + split-K reduce) run on a second stream.  They only feed Parameter.grad, so the
                    # dgrad -> GroupNorm chain does not wait for them, and the small latency-bound kernels of that chain share SMs with wgrad CTAs
 SPLITK = True      # small-M fprop / dgrad launches split their K loop over idle SMs (dp_conv_splitk_workspace_floats)
+# GroupNorm outputs read only by tensor-core fprop / wgrad launches are written already split into fp16 hi / lo' (dp_groupnorm_fwd_split):
+# the convolutions skip their in-kernel split.  DPB200_PRESPLIT=0 plans the fp32 operands instead (A/B runs in one process tree).
+PRESPLIT = os.environ.get("DPB200_PRESPLIT", "1") != "0"
+CONV_X_SPLIT = 4   # dp_conv_args.flags: DP_CONV_X_SPLIT
 ARENA_ALIGN = 64   # floats: every parameter's slice of a flat arena starts on a 256-byte boundary
 
 
@@ -137,6 +141,9 @@ class Plan:
         self._bf_cache: Dict[Tuple[int, int, int], Tuple[torch.Tensor, int]] = {}
         self._bf_packs: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
         self.n_bf16_convs = 0
+        # GroupNorm outputs planned in split form: (buffer address, channel offset, channels) -> (fp16 [rows][2][pitch], pitch)
+        self._split_cache: Dict[Tuple[int, int, int], Tuple[torch.Tensor, int]] = {}
+        self.split_gn: List[str] = []     # shape tags of those GroupNorms, in plan order
         self.model = model
         self.B, self.H, self.W = batch, height, width
         self.dev = torch.device(device)
@@ -361,8 +368,39 @@ class Plan:
             slot = self._fslot[k]
         else:
             slot = self._amax(self.fwd, lambda p=x.ptr: p, x.ld, x.rows, x.C, fwd_key=(x.ptr, x.ld, x.rows, x.C))
-        self._audit(self.fwd, slot, lambda x=x: x.torch())
+        sp = self._split_cache.get((x.t.data_ptr(), x.off, x.C))
+        if sp is not None:     # only the split form is written: check the bound against the operand rebuilt from it
+            self._audit(self.fwd, slot, lambda sp=sp, x=x, slot=slot: self._unsplit(sp, x, slot))
+        else:
+            self._audit(self.fwd, slot, lambda x=x: x.torch())
         return slot
+
+    def _unsplit(self, sp: Tuple[torch.Tensor, int], x: View, slot: int) -> torch.Tensor:
+        """(hi + lo' * 2^-11) / s of a split operand, s = the power of two the kernels derive from the slot (common.cuh scale_up)."""
+        t, pitch = sp
+        bits = int(self._slots[(slot - self._slots.data_ptr()) // 4])
+        E = min(max((bits >> 23) & 0xFF, 14), 254)
+        v = t.view(-1, 2, pitch)[:, :, :x.C].double()
+        return ((v[:, 0] + v[:, 1] * 2.0 ** -11) * 2.0 ** (E - 140)).float()
+
+    def presplit_ok(self, gn_in: View, x: View, out: View, w: nn.Parameter, stride: int = 1, pad: int = 1) -> bool:
+        """Can the GroupNorm gn_in -> x write x in split form for its one consumer, the convolution x -> out with weight w?  Needs the
+        tensor-core fprop and wgrad of that convolution to take a split operand, and one float4 GroupNorm launch (one scale per tensor)."""
+        K, Cin = w.shape[0], w.shape[1]
+        if not (PRESPLIT and self.tc and not self.bf16) or K * Cin < 256:
+            return False
+        if gn_in.C % 4 or gn_in.off % 4 or gn_in.C > self.GN_MAX_C:
+            return False
+        a = L.ConvArgs()
+        a.N, a.H, a.W, a.C = x.N, x.H, x.W, x.C
+        a.P, a.Q, a.K = out.H, out.W, K
+        a.R = w.shape[2] if w.dim() == 4 else 1
+        a.S = w.shape[3] if w.dim() == 4 else 1
+        a.stride, a.pad_t, a.pad_l = stride, pad, pad
+        return self.lib.dp_conv_presplit_eligible(_byref(a)) == 0
+
+    def _split_of(self, x: View) -> Optional[Tuple[torch.Tensor, int]]:
+        return self._split_cache.get((x.t.data_ptr(), x.off, x.C))
 
     def _dy_slot(self, steps: List[Step], v: View) -> int:
         """Consumer side (backward): slot of max|v.grad|.  The writers of v.grad are built later; _finalize_build hands them the slot and
@@ -493,12 +531,17 @@ class Plan:
         if wtc is not None:
             a.w_tc_hi, a.w_tc_lo, a.amax_w = wtc[0].data_ptr(), wtc[1].data_ptr(), wtc[4]
             a.amax_x = self._x_slot(x)
+        xs = self._split_of(x)
+        if xs is not None:
+            assert wtc is not None, "a split operand needs the tensor-core path"
         a.N, a.H, a.W, a.C = x.N, x.H, x.W, x.C
         a.P, a.Q, a.K = out.H, out.W, K
         a.R, a.S, a.stride, a.pad_t, a.pad_l = R, S, stride, pad, pad
-        a.flags = 1 if accumulate_out else 0
+        a.flags = (1 if accumulate_out else 0) | (CONV_X_SPLIT if xs is not None else 0)
         a.splits = 1
         a.x, a.ldx, a.y, a.ldy = x.ptr, x.ld, out.ptr, out.ld
+        if xs is not None:
+            a.x, a.ldx = xs[0].data_ptr(), xs[1]
         a.amax_out = self._out_slot(out)
         a.w = wck.data_ptr()
         a.bias = b.data_ptr() if b is not None else None
@@ -564,7 +607,7 @@ class Plan:
             amax_dy = self._amax(steps, dy_get, dy_ld, out.rows, K) if dy_dense is not None else self._dy_slot(steps, out)
         wa = _copy_args(a)
         wa.amax_y, wa.amax_out = amax_dy, None
-        wa.flags, wa.splits = 0, splits
+        wa.flags, wa.splits = a.flags & CONV_X_SPLIT, splits
         wa.ldy = dy_ld
         wa.rowadd, wa.residual, wa.bias = None, None, None
         self._late.append(lambda wa=wa, g=dy_get, n=ws_name: (setattr(wa, "y", g()), setattr(wa, "workspace", self.sptr(n))))
@@ -664,6 +707,9 @@ class Plan:
         a.R, a.S, a.stride, a.pad_t, a.pad_l = 1, 1, 1, 0, 0
         a.flags, a.splits = 0, 1
         a.x, a.ldx, a.y, a.ldy = x.ptr, x.ld, qkv.ptr, qkv.ld
+        xs = self._split_of(x)
+        if xs is not None:
+            a.flags, a.x, a.ldx = CONV_X_SPLIT, xs[0].data_ptr(), xs[1]
         a.amax_out = self._out_slot(qkv)
         a.w = wck.data_ptr()
         a.bias = bf.data_ptr() if has_bias else None
@@ -693,7 +739,7 @@ class Plan:
             wa.K = inner
             wa.y, wa.ldy = dout.ptr + 4 * i * ip, dout.ld
             wa.amax_y, wa.amax_out = amax_dy, None
-            wa.flags, wa.splits = 0, splits
+            wa.flags, wa.splits = a.flags & CONV_X_SPLIT, splits
             wa.rowadd, wa.residual, wa.bias, wa.workspace = None, None, None, None
             self._late.append(lambda wa=wa, n=ws_name: setattr(wa, "workspace", self.sptr(n)))
             if has_bias:
@@ -814,10 +860,13 @@ class Plan:
 
     GN_MAX_C = 1024      # channels one dp_groupnorm launch handles (256 threads x 4 channel slots); wider tensors are split by groups
 
-    def gn(self, x: View, norm: nn.Module, out: View, silu: bool, dropout_p: float = 0.0, bf16_only: bool = False, groups: Optional[int] = None):
+    def gn(self, x: View, norm: nn.Module, out: View, silu: bool, dropout_p: float = 0.0, bf16_only: bool = False, groups: Optional[int] = None,
+           split_only: bool = False):
         """fwd: out = dropout?(silu?(GN(x))).  Returns the forward argument structs, one per channel part (the backward reuses stats /
         dropout seed).  Groups are independent, so a tensor wider than GN_MAX_C (the LDM's concatenated 1920-channel inputs) runs as
-        k launches over k disjoint ranges of whole groups."""
+        k launches over k disjoint ranges of whole groups.  split_only (every consumer of `out` is a tensor-core fprop / wgrad that
+        takes a split operand, see presplit_ok): write only the fp16 hi / lo' pair the convolutions read, scaled by a bound known in
+        advance (dp_groupnorm_fwd_split); the fp32 tensor is left unwritten."""
         lib = self.lib
         G = groups if groups is not None else norm.num_groups
         parts = 1
@@ -833,6 +882,14 @@ class Plan:
         if bf16_only:   # every consumer of `out` is a bf16 convolution: write the operand directly, skip the fp32 tensor
             yb, ldyb = self._bf_new(out.rows, out.C)
             self._bf_cache[(out.t.data_ptr(), out.off, out.C)] = (yb, ldyb)
+        ys = None
+        if split_only:
+            assert parts == 1 and not bf16_only
+            pitch = lib.dp_tc_weight_row(out.C)     # the packed weights' row length: 128-byte box rows for C > 64
+            ys = torch.zeros((out.rows, 2, pitch), device=self.dev, dtype=torch.float16)   # pad channels stay zero (finite for the MMA)
+            self._keep.append(ys)
+            self._split_cache[(out.t.data_ptr(), out.off, out.C)] = (ys, pitch)
+            self.split_gn.append(f"{out.N}x{out.H}x{out.W}x{out.C}")
         cp, gp = x.C // parts, G // parts
         args = []
         yslot = self._out_slot(out) if not bf16_only else None   # the tensor-core convolutions that read `out` find its slot filled
@@ -845,6 +902,8 @@ class Plan:
             a.x, a.ldx, a.y, a.ldy = x.ptr + 4 * c0, x.ld, out.ptr + 4 * c0, out.ld
             if bf16_only:
                 a.y, a.y_bf16, a.ldyb = None, yb.data_ptr() + 2 * c0, ldyb
+            if split_only:
+                a.y = None
             a.gamma, a.beta = norm.weight.data_ptr() + 4 * c0, norm.bias.data_ptr() + 4 * c0
             stats = torch.empty(2 * x.N * gp, device=self.dev, dtype=torch.float32)
             self._keep.append(stats)
@@ -855,7 +914,10 @@ class Plan:
                 a.dropout_seed_dev = self.dropout_seed_dev.data_ptr()
             self.scratch("gn_ws", (lib.dp_groupnorm_workspace_bytes(a.N, a.HW, a.C, a.G) + 3) // 4)
             self._late.append(lambda a=a: setattr(a, "workspace", self.sptr("gn_ws")))
-            self._rec(self.fwd, lib.dp_groupnorm_fwd, a, "gn fwd")
+            if split_only:
+                self._rec(self.fwd, lambda ref, s, p=ys.data_ptr(), ld=ys.shape[-1]: lib.dp_groupnorm_fwd_split(ref, p, ld, s), a, "gn fwd")
+            else:
+                self._rec(self.fwd, lib.dp_groupnorm_fwd, a, "gn fwd")
             args.append((a, c0))
         return args
 
@@ -903,14 +965,16 @@ class Plan:
         tp = self.new(self.B, 1, 1, Cout)
         has_sc = m.conv_shortcut is not None
         da = lambda: self.sptr("da")
-        g1 = self.gn(x, m.norm1, a1, silu=True, bf16_only=self.conv_bf16_ok(a1, h1, m.conv1.weight))
+        g1 = self.gn(x, m.norm1, a1, silu=True, bf16_only=self.conv_bf16_ok(a1, h1, m.conv1.weight),
+                     split_only=self.presplit_ok(x, a1, h1, m.conv1.weight))
         if self.need_grad:
             self.gn_bwd(g1, x, m.norm1, da, x.C, add2=None if has_sc else self.gradof(out))
         # time_emb_proj(silu(temb)) -> per-image row added in conv1's epilogue; its dY are conv1's per-image sums
         self.conv(self.silu_temb, m.time_emb_proj.weight, m.time_emb_proj.bias, tp, pad=0, dy_dense="seg",
                   dx_into=self.silu_temb)
         self.conv(a1, m.conv1.weight, m.conv1.bias, h1, rowadd=tp, seg_out="seg", dx_scratch="da")
-        g2 = self.gn(h1, m.norm2, a2, silu=True, dropout_p=p_drop, bf16_only=self.conv_bf16_ok(a2, out, m.conv2.weight))
+        g2 = self.gn(h1, m.norm2, a2, silu=True, dropout_p=p_drop, bf16_only=self.conv_bf16_ok(a2, out, m.conv2.weight),
+                     split_only=self.presplit_ok(h1, a2, out, m.conv2.weight))
         if self.need_grad:
             self.gn_bwd(g2, h1, m.norm2, da, Cout)
         if has_sc:
@@ -933,7 +997,8 @@ class Plan:
         if not fuse:
             q, k, v = (self.new(N, H, W, inner) for _ in range(3))
         g = self.gn(x, m.group_norm, xn, silu=False,
-                    bf16_only=(not fuse) and all(self.conv_bf16_ok(xn, q, l.weight, 1, 0) for l in lins))
+                    bf16_only=(not fuse) and all(self.conv_bf16_ok(xn, q, l.weight, 1, 0) for l in lins),
+                    split_only=fuse and self.presplit_ok(x, xn, o, m.to_q.weight, 1, 0))
         if self.need_grad:
             self.gn_bwd(g, x, m.group_norm, lambda xn=xn: self.gradof(xn).ptr, x.C,
                         add2=self.gradof(out) if m.residual_connection else None)
@@ -1311,7 +1376,8 @@ class Plan:
         -> 1x1 proj_out ; + x."""
         h = self.new(x.N, x.H, x.W, m.proj_in.out_channels)
         xn = self.new(x.N, x.H, x.W, x.C)
-        g = self.gn(x, m.norm, xn, silu=False, bf16_only=self.conv_bf16_ok(xn, h, m.proj_in.weight, 1, 0))
+        g = self.gn(x, m.norm, xn, silu=False, bf16_only=self.conv_bf16_ok(xn, h, m.proj_in.weight, 1, 0),
+                    split_only=self.presplit_ok(x, xn, h, m.proj_in.weight, 1, 0))
         if self.need_grad:
             self.gn_bwd(g, x, m.norm, lambda xn=xn: self.gradof(xn).ptr, x.C, add2=self.gradof(out))
         self.conv(xn, m.proj_in.weight, m.proj_in.bias, h, pad=0)

@@ -53,6 +53,11 @@ int dp_tc_available(void);
  * ------------------------------------------------------------------------------------------------ */
 #define DP_CONV_ACCUMULATE 1 /* fprop: y += ; dgrad: dx += (instead of =) */
 #define DP_CONV_FORCE_SIMT 2 /* never take the tensor-core path (testing / odd shapes) */
+/* fprop / wgrad: x is already split for the tensor-core path (dp_groupnorm_fwd_split), fp16 [N][H][W][2][ldx]: per pixel
+ * hi = fp16(s*x) in elements [0, ldx), lo' = fp16((s*x - hi) * 2^11) in [ldx, 2 ldx), s = the power of two of amax_x (see
+ * dp_pack_conv_weight_tc).  ldx counts fp16 ELEMENTS, a multiple of 8, >= C; the pad channels [C, ldx) must hold finite values (zeros).
+ * Such a launch never falls back to the SIMT path (it cannot read the split form): outside dp_conv_presplit_eligible it fails. */
+#define DP_CONV_X_SPLIT 4
 
 typedef struct dp_conv_args {
   int32_t N, H, W, C;
@@ -92,6 +97,9 @@ int dp_conv2d_dgrad(const dp_conv_args* a, dp_stream_t stream);
 long long dp_conv_splitk_workspace_floats(const dp_conv_args* a, int op);
 /* writes split partial sums to a->workspace; dp_conv2d_wgrad_reduce finishes the job */
 int dp_conv2d_wgrad(const dp_conv_args* a, dp_stream_t stream);
+/* DP_OK when both dp_conv2d_fprop and dp_conv2d_wgrad take DP_CONV_X_SPLIT for this geometry (stride 1, 'same' padding, tensor-core
+ * path available; pointers not needed), else DP_ERR_UNSUPPORTED */
+int dp_conv_presplit_eligible(const dp_conv_args* a);
 
 /* dW (OIHW, the nn.Parameter .grad) += sum_splits workspace — fixed order, no atomics (deterministic,
  * ddpm_prune.py:102 accumulates across timesteps, SURVEY.md §0.4).  If `w` and score_out/score_in are given,
@@ -245,6 +253,12 @@ typedef struct dp_gn_args {
 } dp_gn_args;
 size_t dp_groupnorm_workspace_bytes(int32_t N, int32_t HW, int32_t C, int32_t G);
 int dp_groupnorm_fwd(const dp_gn_args* a, dp_stream_t stream);
+/* dp_groupnorm_fwd that also (with a->y == NULL: only) writes its output already split for the tensor-core convolutions, in the
+ * DP_CONV_X_SPLIT layout [N][HW][2][ldys] fp16 (ldys a multiple of 8, >= C; pad channels untouched).  The scale comes from a bound
+ * known before anything is written, B = max|gamma| * sqrt(C/G * HW - 1) + max|beta| (over a group of n values |x - mean| <=
+ * sqrt(n - 1) * std), widened for SiLU and dropout; B goes to a->amax_y (required) in place of the measured max|y|.  Single-launch
+ * float4 path only (C % 4 == 0, 16-byte aligned views): DP_ERR_UNSUPPORTED otherwise. */
+int dp_groupnorm_fwd_split(const dp_gn_args* a, void* y_split, int64_t ldys, dp_stream_t stream);
 int dp_groupnorm_bwd(const dp_gn_args* a, dp_stream_t stream);
 /* dgamma[c] += sum_n fin[n][1][c], dbeta[c] += sum_n fin[n][0][c] (fixed order) — the tail of native_group_norm_backward for a
  * dp_groupnorm_bwd call that was given `fin` */
